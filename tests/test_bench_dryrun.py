@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 import bench
+from vsr_b200._capi import VsrRangeError
 
 
 class _Event:
@@ -57,16 +58,33 @@ class FakeSTTN:
     PROF = ("conv3x3", "conv3x3_residual", "qkv", "score", "softmax", "pv", "encoder", "decoder", "gather", "prepost")
     cuda_stream = 0
 
-    def __init__(self):
+    def __init__(self, out_of_range=False):
         self.launch_count = 0
         self.tickets = 0
+        self.computes = 0
+        self.out_of_range = out_of_range    # logits beyond the single-pass softmax: fetch raises until attn_direct is switched off
+        self.options = {"attn_direct": 1}
+
+    def set_option(self, name, value):
+        self.options[name] = value
 
     def stage(self, frames, mask):
         assert frames[0].dtype == np.uint8 and mask.shape == frames[0].shape[:2]
+        self.staged = (frames, mask)
 
     def compute(self):
         self.launch_count += 700
+        self.computes += 1
         time.sleep(0.001)
+
+    def fetch(self, frames_out):
+        """the staged frames with the number of compute() calls so far written under the mask"""
+        if self.out_of_range and self.options["attn_direct"]:
+            raise VsrRangeError("attention logits beyond the range of the single-pass softmax (attn_direct)")
+        frames, mask = self.staged
+        for o, f in zip(frames_out, frames):
+            o[...] = f
+            o[mask != 0] = self.computes
 
     def sync(self):
         pass
@@ -206,6 +224,36 @@ def test_contract_line_with_cpu_baseline(fake_world, capsys, monkeypatch):
     r = d["roofline"]
     assert r["bound"] == "tensor" and r["unit"] == "TFLOP/s" and r["launches"] == 30 and set(r["in_situ_ms"]) == set(FakeSTTN.PROF)
     assert d["clocks"]["sm_mhz"] == 1800.0
+
+
+def test_dump_outputs_of_the_last_timed_step(fake_world, capsys, tmp_path):
+    """--dump-outputs: float32 samples of the frames fetched after the last of --steps timed steps, within 64 MB, equal from run to run"""
+    runs = []
+    for k in range(2):
+        bench.main(["--steps", "4", "--warmup", "3", "--no-cpu", "--dump-outputs", str(tmp_path / str(k))])
+        d = _line(capsys)
+        assert d["steps"] == 4 and d["config"]["attention"] == "single-pass softmax"
+        runs.append({p.stem: np.load(p) for p in (tmp_path / str(k)).glob("*.npy")})
+    a, b = runs
+    assert set(a) == {"inpainted", "kept"} and all(v.dtype == np.float32 and v.shape[:1] == (bench.CHUNK,) for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    assert np.all(a["inpainted"] == 1 + 3 + 4)                      # fetched after the checked pass, the 3 warm-up and the 4 timed computes
+    S = bench.synthetic()
+    want = bench.output_sample(S.synthetic_clip(bench.CHUNK, bench.H, bench.W, seed=0), S.default_mask(bench.H, bench.W))
+    assert np.array_equal(a["kept"], want["kept"])                  # outside the mask: the input frames
+    for bad in (["--steps", "0"], ["--workload", "lama", "--dump-outputs", str(tmp_path)]):
+        with pytest.raises(SystemExit):
+            bench.main(bad)
+
+
+def test_timed_path_is_the_one_a_caller_gets_when_logits_leave_the_single_pass_range(fake_world, capsys, monkeypatch, tmp_path):
+    """a chunk the single-pass softmax cannot hold: its results are rejected, so the timed steps run (and the dump reads) the exact path"""
+    eng = FakeSTTN(out_of_range=True)
+    monkeypatch.setattr(bench, "make_sttn", lambda dev: (eng, {"w": np.zeros(1, np.float32)}, "stand-in weights"))
+    bench.main(["--steps", "2", "--warmup", "1", "--no-cpu", "--dump-outputs", str(tmp_path)])
+    assert _line(capsys)["config"]["attention"].startswith("score matrix + softmax kernel") and eng.options["attn_direct"] == 0
+    assert np.all(np.load(tmp_path / "inpainted.npy") == 1 + 3 + 2)
 
 
 def test_reference_arm_line(capsys, monkeypatch):

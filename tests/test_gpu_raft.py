@@ -12,8 +12,8 @@ from oracle import raft_oracle as R
 from oracle import sttn_oracle as O
 
 PATH = os.path.join(ROOT, "weights", "propainter", "raft-things.pth")
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not os.path.exists(PATH), reason="raft-things.pth not staged under weights/propainter")]
+pytestmark = pytest.mark.gpu
+needs_raft = pytest.mark.skipif(not os.path.exists(PATH), reason="raft-things.pth not staged under weights/propainter")
 
 
 def check_raft_flows(runtime=None):
@@ -29,6 +29,7 @@ def check_raft_flows(runtime=None):
         assert np.isfinite(got).all() and epe.mean() <= 0.01 and epe.max() <= 0.1, (float(epe.mean()), float(epe.max()))
 
 
+@needs_raft
 def test_raft_flows_vs_oracle(capi):
     check_raft_flows()
 
@@ -59,7 +60,7 @@ def check_image_propagation(runtime=None):
 
 
 def test_image_propagation_vs_oracle(capi):
-    """P5 on the device (gated like the RAFT test)."""
+    """P5 on the device: needs no checkpoint (the flows are the reference's, stored in tests/golden/propainter_real.npz)."""
     check_image_propagation()
 
 
@@ -101,7 +102,7 @@ def test_propainter_pipeline_vs_reference_frames(capi):
     from conftest import GOLDEN
 
     d = os.path.join(ROOT, "weights", "propainter")
-    if not all(os.path.exists(os.path.join(d, f)) for f in ("ProPainter.pth", "recurrent_flow_completion.pth")):
+    if not all(os.path.exists(os.path.join(d, f)) for f in ("ProPainter.pth", "recurrent_flow_completion.pth", "raft-things.pth")):
         pytest.skip("ProPainter weights not staged")
     sys.path.insert(0, os.path.join(ROOT, "tools"))
     from make_golden_propainter import inputs
@@ -119,8 +120,7 @@ def test_propainter_pipeline_vs_reference_frames(capi):
 
 
 def test_batched_detection_equals_single_frames(capi):
-    """`TextDetector.probability_maps` (several sampled frames per launch): written after the GPU budget was spent, gated like the rest of this
-    file; bar: every frame's map equals its single-frame map to fp16 noise (the scales may differ between the two programs)."""
+    """`TextDetector.probability_maps` (several sampled frames per launch), gated on the detector model; bar: every frame's map equals its single-frame map to fp16 noise (the scales may differ between the two programs)."""
     import cv2
 
     model = os.path.join(ROOT, "weights", "V5", "ch_det")

@@ -220,9 +220,43 @@ def test_config2_whole_chunk_vs_reference_golden(real_engine):
     assert bias < 0.1, f"mean error per masked sample {bias:.3f} grey levels (PSNR {psnr:.2f} dB)"   # every frame's mean error: < 0.1 grey levels
 
 
-def test_full_size_properties_1080p(real_engine):
-    """BASELINE config 2 at full size (one 50-frame chunk): size-independent properties."""
-    eng, _ = real_engine
+@pytest.fixture(scope="module")
+def rand_engine_1080p(capi):
+    """Seeded random-init weights (those bench.py runs without a checkpoint) on an engine of its own: their logits leave the range of the
+    single-pass softmax on the 1080p chunk, and the switch to the exact path must not carry over to the engine the other tests share."""
+    from vsr_b200 import STTNInpaint
+
+    w = O.random_weights(0)
+    return STTNInpaint("cuda:0", {k: v.numpy() for k, v in w.items()}), w
+
+
+def test_config2_whole_chunk_vs_oracle_random_weights(rand_engine_1080p):
+    """BASELINE config 2 at full size with the seeded random-init weights: the chunk bench.py times, on the attention path its timed
+    steps take with those weights, against the oracle's `STTNInpaint.__call__` (oracle/sttn_oracle.py, pinned to the reference's outputs
+    by tests/test_oracle_golden.py); rows outside the strip and unmasked pixels bit-exact."""
+    eng, w = rand_engine_1080p
+    H, W, T = 1080, 1920, 50
+    frames = O.synthetic_clip(T, H, W, seed=0)
+    mask = O.default_mask(H, W)
+    out = eng(frames, mask)
+    want = O.sttn_call(w, frames, mask)
+    _check_images([o[720:] for o in out], [x[720:] for x in want])
+    m = mask > 127
+    for o, f in zip(out, frames):
+        assert np.array_equal(o[:720], f[:720]) and np.array_equal(o[~m], f[~m])
+
+
+def test_full_size_properties_1080p(rand_engine_1080p):
+    """BASELINE config 2 at full size (one 50-frame chunk): size-independent properties, seeded random-init weights."""
+    _full_size_properties(rand_engine_1080p[0])
+
+
+def test_full_size_properties_1080p_real_weights(real_engine):
+    """The same properties with the reference checkpoint, whose logits stay on the single-pass softmax path."""
+    _full_size_properties(real_engine[0])
+
+
+def _full_size_properties(eng):
     H, W, T = 1080, 1920, 50
     frames = O.synthetic_clip(T, H, W, seed=0)
     mask = O.default_mask(H, W)

@@ -9,9 +9,11 @@ import pytest
 from conftest import ROOT
 
 DIR = os.path.join(ROOT, "weights", "propainter")
-pytestmark = [pytest.mark.slow,
-              pytest.mark.skipif(not all(os.path.exists(os.path.join(DIR, f)) for f in ("raft-things.pth", "recurrent_flow_completion.pth")),
-                                 reason="ProPainter weights not staged under weights/propainter")]
+pytestmark = pytest.mark.slow
+
+
+def _needs(name):
+    return pytest.mark.skipif(not os.path.exists(os.path.join(DIR, name)), reason=f"{name} not staged under weights/propainter")
 
 
 @pytest.fixture(scope="module")
@@ -26,6 +28,7 @@ def hybrid():
     _capi._lib = saved
 
 
+@_needs("raft-things.pth")
 def test_raft_stage_check(hybrid):
     import test_gpu_raft as G
 
@@ -38,6 +41,7 @@ def test_image_propagation_stage_check(hybrid):
     G.check_image_propagation(hybrid())
 
 
+@_needs("recurrent_flow_completion.pth")
 def test_flow_completion_stage_check(hybrid):
     import test_gpu_raft as G
 
